@@ -57,7 +57,13 @@ def parse():
                     help="wall-clock budget of the CPU arm; whole epochs are dropped (never shortened) beyond it")
     ap.add_argument("--matmul", default="tc3", choices=["fp32", "tf32x3", "tc3"],
                     help="MLP GEMM path: tc3 = hand-written tcgen05 3xTF32 kernel on the 256-wide layers (default), fp32 = cuBLAS SIMT everywhere, tf32x3 = 3 cuBLAS TF32 GEMMs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last device-timed step computed (rollout sample, "
+                         "advantages, returns, normaliser state, parameters, logged scalars) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -603,6 +609,32 @@ def secondary_measurements(args, device):
 
 
 SETTLE_EPOCHS = 30        # untimed epochs between the W warm-up steps and the first timed leg (see run_ours)
+DUMP_ENVS = 1024          # envs sampled (fixed seed) for --dump-outputs: ~25 MB whatever --envs-per-gpu is
+
+
+def dump_outputs(path, agent, buf, env):
+    """--dump-outputs: what the last timed epoch computed, as a caller of the collector + PPO update receives it.
+    The rollout (T, N, .) arrays, its advantages and returns on a fixed seeded sample of DUMP_ENVS envs (their
+    indices in env_sample.npy); the observation normaliser's state; the flat pf|vf parameters after the update; every
+    logged scalar of every minibatch update.  Runs before anything else touches the buffer."""
+    import re
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    n = buf.env_nums
+    cols = np.sort(np.random.RandomState(0).choice(n, min(n, DUMP_ENVS), replace=False))
+    idx = torch.as_tensor(cols, device=agent.device)
+    out = {"env_sample": cols, "params": agent.opt.data}
+    for k in ("obs", "next_obs", "acts", "rewards", "values", "terminals", "time_limits", "advs", "estimate_returns"):
+        out[k] = getattr(buf, "_" + k).index_select(1, idx)
+    nrm = env._obs_normalizer
+    out.update(obs_norm_mean=nrm._mean, obs_norm_var=nrm._var, obs_norm_count=nrm._count)
+    infos = agent._flush_infos(agent._mb_state["U"])
+    for key in infos[0]:
+        out["info_" + re.sub(r"[^A-Za-z0-9_.-]", "_", key)] = np.array([i[key] for i in infos], dtype=np.float64)
+    for name, v in out.items():
+        a = v.detach().cpu().numpy() if torch.is_tensor(v) else np.asarray(v)
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
 
 
 def run_ours(args):
@@ -687,6 +719,8 @@ def run_ours(args):
     t_dev = ctx.max_over_ranks(marks[0].elapsed_time(marks[-1]) * 1e-3)
     step_ms = [round(marks[k].elapsed_time(marks[k + 1]), 3) for k in range(args.steps)]    # this rank's steps
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, agent, buf, env)
 
     value = frames_per_step * args.steps / t_dev
     e2e_value = frames_per_step * args.steps / t_e2e

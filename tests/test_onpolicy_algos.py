@@ -1,20 +1,32 @@
-"""A2C, V-MPO and TRPO on the device against the EXECUTED reference (oracle/_ref or /root/reference behind oracle/shims,
-torch CPU): same initial weights (state_dict copied from the reference's networks), the same explicit batches through
-`update(batch)` -- the reference's own entry point -- then the logged scalars of every update and the parameters after
-the last one are compared.  SURVEY.md 8(f).4.
+"""A2C, V-MPO and TRPO on the device against the reference (torch CPU): the reference's agents were run on the
+explicit batches below through `update(batch)` -- the reference's own entry point -- and their initial weights, the
+logged scalars of every update and the parameters after the updates are stored in tests/golden/onpolicy_algos.npz
+(`python -m oracle.make_golden onpolicy` regenerates it where the reference is importable).  The device agents start
+from the stored weights, take the same batches and must reproduce the stored scalars and parameters.  SURVEY.md 8(f).4.
 
 Stated tolerances (fp32 device kernels vs torch-CPU fp32): logged scalars rtol 2e-3 + atol 2e-4 (TRPO policy loss /
 KL-driven quantities 5e-3), parameters atol 2e-4 (TRPO: 1e-3 of the step, the conjugate-gradient solve amplifies
 rounding).  The device epoch loop (captured graphs) is checked against the eager `update` path of the same agent.
 """
+import json
+import os
+
 import numpy as np
 import pytest
 
-from oracle import reference_loader
-
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not reference_loader.available(), reason="no copy of the reference")]
+pytestmark = pytest.mark.gpu
 
 O, A, HID = 11, 3, (32, 32)
+KW = {"a2c": dict(plr=1e-3, vlr=1e-3, entropy_coeff=0.01),
+      "vmpo": dict(plr=1e-3, vlr=1e-3, opt_epochs=2, alpha_eps=0.01),
+      "trpo": dict(plr=3e-4, vlr=1e-3, max_kl=0.01, cg_damping=0.1, cg_iters=10, residual_tol=1e-10, entropy_coeff=0.01,
+                   v_opt_times=2)}
+TRPO_LEADS = [None, (8, 16)]
+
+
+@pytest.fixture(scope="module")
+def g(golden_dir):
+    return np.load(os.path.join(golden_dir, "onpolicy_algos.npz"))
 
 
 class _NullLogger:
@@ -50,29 +62,23 @@ def _batches(n, B, seed, lead=None):
     return out
 
 
-def _reference_agent(kind, tmp_path, **algo_kw):
+def _stored(g, tag, names=("pf", "vf")):
+    """{net.key: array} of what _params() returned for the reference agent at `tag`."""
+    pre = tag + "_"
+    return {k[len(pre):]: g[k].astype(np.float64) for k in g.files
+            if k.startswith(pre) and k[len(pre):].split(".")[0] in names}
+
+
+def _stored_infos(g, tag):
+    return json.loads(str(g[tag + "_infos"]))
+
+
+def _load(net, params, name):
     import torch
-    reference_loader.load()                  # puts the gym / tensorboardX shims on sys.path
-    import gym
-    import torchrl.networks as networks
-    import torchrl.policies as policies
-    from torchrl.algo import A2C, TRPO, VMPO
-
-    class Env:
-        action_space = gym.spaces.Box(-np.ones(A), np.ones(A))
-        observation_space = gym.spaces.Box(-np.ones(O), np.ones(O))
-    torch.manual_seed(3)
-    net = dict(hidden_shapes=list(HID), append_hidden_shapes=[], base_type=networks.MLPBase, activation_func=torch.nn.Tanh)
-    pf = policies.GuassianContPolicyBasicBias(input_shape=O, output_shape=A, tanh_action=True, **net)
-    vf = networks.Net(input_shape=(O,), output_shape=1, **net)
-    cls = {"a2c": A2C, "vmpo": VMPO, "trpo": TRPO}[kind]
-    agent = cls(pf=pf, vf=vf, env=Env(), replay_buffer=None, collector=_Col(), logger=_NullLogger(), discount=0.99,
-                num_epochs=10, batch_size=64, gae=True, device="cpu", save_dir=str(tmp_path), shuffle=True, tau=0.95,
-                **algo_kw)
-    return agent
+    net.load_state_dict({k[len(name) + 1:]: torch.from_numpy(v) for k, v in params.items() if k.startswith(name + ".")})
 
 
-def _device_agent(kind, ref_agent, **algo_kw):
+def _device_agent(kind, init):
     import torch
     import torchrl_b200.networks as networks
     import torchrl_b200.policies as policies
@@ -85,12 +91,12 @@ def _device_agent(kind, ref_agent, **algo_kw):
     net = dict(hidden_shapes=list(HID), append_hidden_shapes=[], base_type=networks.MLPBase, activation_func=torch.nn.Tanh)
     pf = policies.GuassianContPolicyBasicBias(input_shape=O, output_shape=A, tanh_action=True, **net)
     vf = networks.Net(input_shape=(O,), output_shape=1, **net)
-    pf.load_state_dict(ref_agent.pf.state_dict())
-    vf.load_state_dict(ref_agent.vf.state_dict())
+    _load(pf, init, "pf")
+    _load(vf, init, "vf")
     cls = {"a2c": A2C, "vmpo": VMPO, "trpo": TRPO}[kind]
     return cls(pf=pf, vf=vf, env=Env(), replay_buffer=None, collector=_Col(), logger=_NullLogger(), discount=0.99,
                num_epochs=10, batch_size=64, gae=True, device="cuda:0", save_dir=None, shuffle=True, tau=0.95,
-               use_cuda_graph=False, **algo_kw)
+               use_cuda_graph=False, **KW[kind])
 
 
 def _params(agent, names=("pf", "vf")):
@@ -112,68 +118,59 @@ def _compare_infos(mine, ref, rtol=2e-3, atol=2e-4, skip=()):
             assert abs(m[k] - v) <= rtol * abs(v) + atol, (u, k, m[k], v)
 
 
-def test_a2c_update_matches_reference(tmp_path):
-    kw = dict(plr=1e-3, vlr=1e-3, entropy_coeff=0.01)
-    ref = _reference_agent("a2c", tmp_path, **kw)
-    mine = _device_agent("a2c", ref, **kw)
+def test_a2c_update_matches_reference(g):
+    mine = _device_agent("a2c", _stored(g, "init"))
     batches = _batches(4, 64, 0)
-    r_infos = [ref.update(b) for b in batches]
     m_infos = [mine.update(b) for b in batches]
-    _compare_infos(m_infos, r_infos)
-    pr, pm = _params(ref), _params(mine)
+    _compare_infos(m_infos, _stored_infos(g, "a2c"))
+    pr, pm = _stored(g, "a2c_final"), _params(mine)
+    assert pr.keys() == pm.keys()
     for k in pr:
         np.testing.assert_allclose(pm[k], pr[k], atol=2e-4, err_msg=k)
 
 
-def test_vmpo_update_matches_reference(tmp_path):
-    kw = dict(plr=1e-3, vlr=1e-3, opt_epochs=2, alpha_eps=0.01)
-    ref = _reference_agent("vmpo", tmp_path, **kw)
-    mine = _device_agent("vmpo", ref, **kw)
+def test_vmpo_update_matches_reference(g):
+    mine = _device_agent("vmpo", _stored(g, "init"))
     batches = _batches(4, 64, 1)
-    r_infos = [ref.update(b) for b in batches]
     m_infos = [mine.update(b) for b in batches]
-    _compare_infos(m_infos, r_infos)
-    pr, pm = _params(ref), _params(mine)
+    _compare_infos(m_infos, _stored_infos(g, "vmpo"))
+    pr, pm = _stored(g, "vmpo_final"), _params(mine)
+    assert pr.keys() == pm.keys()
     for k in pr:
         np.testing.assert_allclose(pm[k], pr[k], atol=2e-4, err_msg=k)
-    assert abs(float(mine.dual[0]) - float(ref.eta)) < 2e-4 and abs(float(mine.dual[1]) - float(ref.alpha)) < 2e-4
+    eta, alpha = g["vmpo_dual"]
+    assert abs(float(mine.dual[0]) - eta) < 2e-4 and abs(float(mine.dual[1]) - alpha) < 2e-4
 
 
-@pytest.mark.parametrize("lead", [None, (8, 16)])
-def test_trpo_update_matches_reference(tmp_path, lead):
+@pytest.mark.parametrize("lead", TRPO_LEADS)
+def test_trpo_update_matches_reference(g, lead):
     """Flat (B, .) batches (per-sample KL) and the (T, N, .) whole-rollout form the reference's update_per_epoch
     passes (its KL sums over the env axis: the N / act_dim quirk)."""
-    kw = dict(plr=3e-4, vlr=1e-3, max_kl=0.01, cg_damping=0.1, cg_iters=10, residual_tol=1e-10, entropy_coeff=0.01,
-              v_opt_times=2)
-    ref = _reference_agent("trpo", tmp_path, **kw)
-    mine = _device_agent("trpo", ref, **kw)
+    tag = "trpo_%s" % ("flat" if lead is None else "x".join(map(str, lead)))
+    mine = _device_agent("trpo", _stored(g, "init"))
     # actions the policy could have produced (log-probs of arbitrary actions underflow exp() in the reference's ratio)
-    import torch
     batches = _batches(2, 128, 2, lead)
-    for b in batches:
-        with torch.no_grad():
-            o = torch.as_tensor(b["obs"], dtype=torch.float32)
-            mean, std, _ = ref.pf(o)
-            b["acts"] = torch.tanh(mean + std * torch.randn_like(mean)).numpy().astype(np.float64)
-    p0 = _params(ref, ("pf",))
-    for b in batches:
-        r_info = ref.update(b)
+    for i, b in enumerate(batches):
+        b["acts"] = g["%s_acts%d" % (tag, i)]
+    p0 = _stored(g, "init", ("pf",))
+    for i, b in enumerate(batches):
         m_info = mine.update(b)
-        _compare_infos([m_info], [r_info], rtol=5e-3, atol=5e-4)
-        pr, pm = _params(ref, ("pf",)), _params(mine, ("pf",))
+        _compare_infos([m_info], _stored_infos(g, "%s_u%d" % (tag, i)), rtol=5e-3, atol=5e-4)
+        pr, pm = _stored(g, "%s_u%d" % (tag, i), ("pf",)), _params(mine, ("pf",))
+        assert pr.keys() == pm.keys()
         step = max(np.abs(pr[k] - p0[k]).max() for k in pr)
         assert step > 1e-5, "the reference took no step: the test would be vacuous"
         for k in pr:
             np.testing.assert_allclose(pm[k], pr[k], atol=2e-2 * step + 1e-5, err_msg=k)
         # continue both from the SAME parameters so that one update's rounding does not leak into the next
-        mine.pf.load_state_dict(ref.pf.state_dict())
+        _load(mine.pf, pr, "pf")
         p0 = pr
     flat = [dict(obs=b["obs"].reshape(-1, O), estimate_returns=b["estimate_returns"].reshape(-1, 1)) for b in batches]
-    for b in flat:
-        r_info = ref.update_vf(b)
+    for i, b in enumerate(flat):
         m_info = mine.update_vf(b)
-        _compare_infos([m_info], [r_info])
-    pr, pm = _params(ref, ("vf",)), _params(mine, ("vf",))
+        _compare_infos([m_info], _stored_infos(g, "%s_v%d" % (tag, i)))
+    pr, pm = _stored(g, tag + "_final", ("vf",)), _params(mine, ("vf",))
+    assert pr.keys() == pm.keys()
     for k in pr:
         np.testing.assert_allclose(pm[k], pr[k], atol=2e-4, err_msg=k)
 

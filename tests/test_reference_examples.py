@@ -15,7 +15,7 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_EXAMPLES = os.path.join(ROOT, "oracle", "_ref", "examples")
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_EXAMPLES), reason="oracle/_ref not built")
+needs_ref = pytest.mark.skipif(not os.path.isdir(REF_EXAMPLES), reason="oracle/_ref not built")
 
 
 def _run_reference_example(script, cfg_name, patch, nenv, tmp_path, extra_check=None):
@@ -56,6 +56,7 @@ def _small_off_policy(c, n=32):
 
 
 @pytest.mark.gpu
+@needs_ref
 def test_reference_ppo_example_runs_unmodified(tmp_path):
     def patch(c):
         _small_on_policy(c, "ppo")
@@ -69,6 +70,7 @@ def test_reference_ppo_example_runs_unmodified(tmp_path):
 
 
 @pytest.mark.gpu
+@needs_ref
 def test_reference_twin_sac_q_example_runs_unmodified(tmp_path):
     work, header = _run_reference_example("twin_sac_q_continuous_vec.py", "twin_sac_q_synth_ant.json", _small_off_policy, 32,
                                            tmp_path)
@@ -78,6 +80,7 @@ def test_reference_twin_sac_q_example_runs_unmodified(tmp_path):
 
 
 @pytest.mark.gpu
+@needs_ref
 def test_reference_td3_example_runs_unmodified(tmp_path):
     work, header = _run_reference_example("td3_continuous_vec.py", "td3_synth_halfcheetah.json", _small_off_policy, 32,
                                            tmp_path)
@@ -86,6 +89,7 @@ def test_reference_td3_example_runs_unmodified(tmp_path):
 
 
 @pytest.mark.gpu
+@needs_ref
 def test_reference_ddpg_example_runs_unmodified(tmp_path):
     work, header = _run_reference_example("ddpg_continuous_vec.py", "ddpg_synth_halfcheetah.json", _small_off_policy, 32,
                                            tmp_path)
@@ -93,6 +97,7 @@ def test_reference_ddpg_example_runs_unmodified(tmp_path):
 
 
 @pytest.mark.gpu
+@needs_ref
 def test_reference_a2c_example_runs_unmodified(tmp_path):
     def patch(c):
         _small_on_policy(c, "a2c")
